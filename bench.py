@@ -2,7 +2,7 @@
 """bench.py -- the GAN training step of the reference's hot path on B200, one JSON line per run.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|stock|reference]
-                    [--config dcgan|wgan_gp|pix2pix|cyclegan]
+                    [--config dcgan|wgan_gp|pix2pix|cyclegan] [--dump-outputs DIR]
 
 Default: BASELINE configs[1] -- DCGAN 64x64, batch 128 per GPU, the full G+D step of dcgan.py:146-183, images/sec.
 N > 1 is launched by torchrun (one rank per GPU, NCCL, weak scaling).  Rank 0 prints ONE JSON line.
@@ -61,7 +61,11 @@ def parse_args():
     ap.add_argument("--no-gpu-reference", action="store_true")
     ap.add_argument("--no-roofline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="eager step loop (debugging)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the losses of the last timed step and the state of the networks it trained to DIR/*.npy")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours or stock: the reference leg shrinks its batch to fit a time budget")
     if a.steps is None:
         a.steps = {"dcgan": 50, "wgan_gp": 200, "pix2pix": 20, "cyclegan": 10}[a.config]
     return a
@@ -303,7 +307,8 @@ def cublas_tf32_tflops(torch):
 # the step under test
 # ---------------------------------------------------------------------------------------------------
 def build_job(torch, config, stock, dev, world, rank):
-    """Returns (step_fn(*inputs) -> tensor of losses, host input pools, D2H bytes per step)."""
+    """Returns (step_fn(*inputs) -> tensor of losses, host input pools, D2H bytes per step, {name: network the step
+    trains})."""
     import itertools
     from b200gan import optim, train, zoo
     cfg = CONFIGS[config]
@@ -342,6 +347,7 @@ def build_job(torch, config, stock, dev, world, rank):
             gl, dl, _ = train.dcgan_step(g, d, og, od, imgs, z, loss, valid, fake, rg, rd)
             return torch.stack([gl, dl])
         pools = [images(1), [torch.randn(B, LATENT, generator=gen).pin_memory() for _ in range(pool_n)]]
+        nets = {"generator": g, "discriminator": d}
     elif config == "wgan_gp":
         g = zoo.WGANGPGenerator((1, img, img), nn=ns).to(dev)
         d = zoo.WGANGPDiscriminator((1, img, img), nn=ns).to(dev)
@@ -354,6 +360,7 @@ def build_job(torch, config, stock, dev, world, rank):
             return torch.stack([dl, gp])
         pools = [images(1), [torch.randn(B, LATENT, generator=gen).pin_memory() for _ in range(pool_n)],
                  [torch.rand(B, 1, 1, 1, generator=gen).pin_memory() for _ in range(pool_n)]]
+        nets = {"discriminator": d}
     elif config == "pix2pix":
         g, d = zoo.GeneratorUNet(nn=ns).to(dev), zoo.Pix2PixDiscriminator(nn=ns).to(dev)
         g.apply(zoo.weights_init_normal)
@@ -365,6 +372,7 @@ def build_job(torch, config, stock, dev, world, rank):
             lg, ld = train.pix2pix_step(g, d, og, od, a, b, reduce_g=rg, reduce_d=rd)
             return torch.stack([lg, ld])
         pools = [images(3), images(3)]
+        nets = {"generator": g, "discriminator": d}
     else:
         shape = (3, img, img)
         nets = [zoo.GeneratorResNet(shape, 9, nn=ns), zoo.GeneratorResNet(shape, 9, nn=ns),
@@ -382,12 +390,31 @@ def build_job(torch, config, stock, dev, world, rank):
             lg, ld = train.cyclegan_step(*nets, og, oa, ob, a, b, None, None, reduce_g=rg, reduce_d_a=ra, reduce_d_b=rb)
             return torch.stack([lg, ld])
         pools = [images(3), images(3)]
-    return step, pools, 8
+        nets = dict(zip(("G_AB", "G_BA", "D_A", "D_B"), nets))
+    return step, pools, 8, nets
 
 
-def time_job(torch, dist, args, stock, dev, world, rank, local, steps, warmup, clocks=False):
+DUMP_FLOATS = 3_000_000  # per trained network: the four of CycleGAN stay under 64 MB
+
+
+def snapshot_outputs(torch, losses, nets):
+    """What a step hands back: its losses, and the state (weights, running statistics) of every network it trains,
+    flattened in state_dict order.  A network of more than DUMP_FLOATS values is cut to a fixed, seeded sample.
+    Split reductions add their partial sums in no fixed order, so two runs agree to rounding, not bit for bit."""
+    out = {"losses": losses.detach().float().cpu().numpy()}
+    for name, net in nets.items():
+        flat = torch.cat([v.detach().float().flatten() for v in net.state_dict().values() if v.is_floating_point()])
+        flat = flat.cpu()
+        if flat.numel() > DUMP_FLOATS:
+            pick = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_FLOATS]
+            flat = flat[pick.sort().values]
+        out[name] = flat.numpy()
+    return out
+
+
+def time_job(torch, dist, args, stock, dev, world, rank, local, steps, warmup, clocks=False, dump=False):
     from b200gan import _lib, train
-    step, pools, d2h = build_job(torch, args.config, stock, dev, world, rank)
+    step, pools, d2h, nets = build_job(torch, args.config, stock, dev, world, rank)
     pool_n = len(pools[0])
     dev_pools = [[t.to(dev) for t in p] for p in pools]
     torch.manual_seed(99 + rank)  # dropout streams differ per rank
@@ -430,6 +457,7 @@ def time_job(torch, dist, args, stock, dev, world, rank, local, steps, warmup, c
     clk = sampler.stop() if (sampler and rank == 0) else None
     ms = e0.elapsed_time(e1)
     losses = out.tolist()
+    outputs = snapshot_outputs(torch, out, nets) if dump else None  # before the e2e leg trains further
     # e2e: host buffers in, losses out, every step
     for i in range(3):
         runner(*[p[i % pool_n] for p in pools])
@@ -448,7 +476,7 @@ def time_job(torch, dist, args, stock, dev, world, rank, local, steps, warmup, c
     ms, ms_e2e = t.tolist()
     h2d = sum(p[0].numel() * 4 for p in pools)
     res = dict(ms_per_step=ms / steps, ms_per_step_e2e=ms_e2e / steps, losses=losses, clocks=clk, h2d=h2d, d2h=d2h,
-               calls_per_step=calls_per_step, graph_error=graph_error)
+               calls_per_step=calls_per_step, graph_error=graph_error, outputs=outputs)
     del runner, step
     return res
 
@@ -495,10 +523,16 @@ def run_gpu(args):
                    "e2e_ms_per_step": r["ms_per_step_e2e"]}
         torch.cuda.empty_cache()
     set_stock_flags(stock)
-    res = time_job(torch, dist, args, stock, dev, world, rank, local, args.steps, args.warmup, clocks=True)
+    res = time_job(torch, dist, args, stock, dev, world, rank, local, args.steps, args.warmup, clocks=True,
+                   dump=bool(args.dump_outputs) and rank == 0)
     if rank != 0:
         _finish(world)
         return
+    if args.dump_outputs:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in res["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), arr)
 
     hbm_peak, bf16_peak, peak_src = measured_peaks()
     tf32_peak = bf16_peak / 2.0  # kind::tf32 issues at half the kind::f16 rate (guide: 1.13 vs 2.25 PF nominal)

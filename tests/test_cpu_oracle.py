@@ -212,18 +212,18 @@ def test_wgan_gp_oracle_and_closed_form_against_reference_golden(golden_dir):
     assert abs(np.linalg.norm(dw2) - fix["dW2_norm"]) < 1e-5 * fix["dW2_norm"]
 
 
-REF = "/root/reference/implementations"
+SCRIPTS = os.path.join(ROOT, "tests", "scripts")
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present on this box")
 def test_launcher_runs_unmodified_gan_script_on_cpu_config0():
-    """BASELINE config 0: implementations/gan/gan.py, 28x28 synthetic, batch 64, CPU -- the unmodified script
-    under the launcher with the drop-in classes patched in (MLP: stock ops through the same classes) prints the
-    same losses as the stock run."""
+    """BASELINE config 0: an MLP GAN script in the reference's idiom (tests/scripts/mini_mlpgan), 28x28 synthetic,
+    batch 64, CPU -- the unmodified script under the launcher with the drop-in classes patched in (MLP: stock ops
+    through the same classes) prints the same losses as the stock run."""
     from b200gan import launch
-    args = ["--n_epochs", "1", "--batch_size", "64", "--sample_interval", "1000"]
-    ours = launch.run(os.path.join(REF, "gan", "gan.py"), args, iters=3, seed=0, stock=False, quiet=True)
-    stock = launch.run(os.path.join(REF, "gan", "gan.py"), args, iters=3, seed=0, stock=True, quiet=True)
+    script = os.path.join(SCRIPTS, "mini_mlpgan", "mini_mlpgan.py")
+    args = ["--epochs", "1", "--batch_size", "64"]
+    ours = launch.run(script, args, iters=3, seed=0, stock=False, quiet=True)
+    stock = launch.run(script, args, iters=3, seed=0, stock=True, quiet=True)
     lines = [l for l in ours["__b200_stdout__"].splitlines() if "[D loss" in l]
     assert len(lines) == 3
     assert ours["__b200_stdout__"] == stock["__b200_stdout__"]
@@ -233,15 +233,19 @@ def test_launcher_runs_unmodified_gan_script_on_cpu_config0():
     assert not isinstance(stock["generator"].model, bnn.Sequential)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present on this box")
 def test_launcher_builds_dcgan_with_drop_in_modules():
+    """A DCGAN-style script in the reference's idiom (tests/scripts/mini_convgan), built under the launcher: the
+    drop-in classes are patched in and draw the same initial weights as the stock run of the same script."""
     from b200gan import launch, nn as bnn
-    g = launch.run(os.path.join(REF, "dcgan", "dcgan.py"), ["--n_epochs", "0", "--img_size", "32"], iters=1, seed=0,
-                   quiet=True)
-    gen, ref = g["generator"], ref_models.build_dcgan(32, seed=0)[0]
-    assert isinstance(gen.conv_blocks, bnn.Sequential) and isinstance(gen.conv_blocks[2], bnn.Conv2d)
-    for k, v in ref.state_dict().items():   # same init draws as the stock run of the same script
-        assert torch.equal(gen.state_dict()[k], v), k
+    script = os.path.join(SCRIPTS, "mini_convgan", "mini_convgan.py")
+    args = ["--epochs", "0", "--side", "32"]
+    ours = launch.run(script, args, iters=1, seed=0, quiet=True)
+    stock = launch.run(script, args, iters=1, seed=0, stock=True, quiet=True)
+    gen, ref = ours["G"], stock["G"]
+    assert isinstance(gen.body, bnn.Sequential) and isinstance(gen.body[2], bnn.Conv2d)
+    assert not isinstance(ref.body, bnn.Sequential)
+    for k, v in ref.state_dict().items():
+        assert torch.equal(gen.state_dict()[k].cpu(), v.cpu()), k
 
 
 def test_pix2pix_and_cyclegan_oracle_against_reference_golden(golden_dir):
