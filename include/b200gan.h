@@ -194,6 +194,18 @@ int b200gan_norm_apply(const b200gan_norm_desc *d, const float *x, const float *
 int b200gan_norm_bwd(const b200gan_norm_desc *d, const float *dy, const float *x, const float *y,
                      const float *mean_rstd, const float *scale_shift, const float *gamma, double *sums, float *dx,
                      float *dgamma_dbeta, void *stream);
+/* Double backward of training-mode BatchNorm2d (per_sample == 0 only; InstanceNorm returns an error) with an optional
+ * fused LeakyReLU / ReLU: the derivative of b200gan_norm_bwd's outputs (dx, dgamma, dbeta) w.r.t. its inputs, for the
+ * gradient penalty of a BatchNorm critic (autograd.grad(..., create_graph=True)).
+ * Inputs: dy and x as given to b200gan_norm_bwd, u = dL/d(dx), mean_rstd, scale_shift (required for a fused activation:
+ * the mask is recomputed from the sign of x * scale + shift; may be NULL without one), gamma (NULL = 1),
+ * gg_gamma = dL/d(dgamma) and gg_beta = dL/d(dbeta) [C] (each may be NULL = 0).
+ * sums[5][C] fp64 workspace: zero on entry, handed back zeroed.
+ * Outputs, all overwritten: gx = dL/dx and gdy = dL/d(dy) [N][HW][C]; dgamma [C] = dL/dgamma (may be NULL).
+ * round_tf32 is ignored: both outputs are gradients that autograd sums with other terms, not conv operands. */
+int b200gan_norm_bwd_bwd(const b200gan_norm_desc *d, const float *dy, const float *x, const float *u,
+                         const float *mean_rstd, const float *scale_shift, const float *gamma, const float *gg_gamma,
+                         const float *gg_beta, double *sums, float *gx, float *gdy, float *dgamma, void *stream);
 
 /* ---- Generator tail: BatchNorm2d -> LeakyReLU/ReLU -> Conv2d(C, K<=3, 3, 1, 1) -> Tanh, fused -------------- */
 /* Replaces the module run dcgan.py:60-63

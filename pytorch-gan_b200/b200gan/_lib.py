@@ -81,6 +81,7 @@ SIGNATURES = {
     "b200gan_norm_finalize": (c_i32, [_P(NormDesc), c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "b200gan_norm_apply": (c_i32, [_P(NormDesc), c_vp, c_vp, c_vp, c_vp]),
     "b200gan_norm_bwd": (c_i32, [_P(NormDesc), c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "b200gan_norm_bwd_bwd": (c_i32, [_P(NormDesc)] + [c_vp] * 13),
     "b200gan_tail_supported": (c_i32, [_P(TailDesc)]),
     "b200gan_tail_fprop": (c_i32, [_P(TailDesc), c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
     "b200gan_tail_bwd_workspace_bytes": (c_sz, [_P(TailDesc)]),

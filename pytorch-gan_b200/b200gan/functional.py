@@ -125,6 +125,7 @@ class ConvFn(torch.autograd.Function):
     def forward(ctx, x, weight, bias, chan_scale, spec: ConvSpec, cache: PackCache):
         ops._require_cuda(x, "conv input")
         ops._require_cuda(weight, "conv weight")
+        ctx.in_nchw = not ops.is_cl(x)
         x = _as_cl(x)
         g, _ = ops.make_geom(tuple(x.shape), tuple(weight.shape), spec.stride, spec.pads, spec.pad_mode, spec.up,
                              spec.transposed)
@@ -269,6 +270,8 @@ def _conv_backward_differentiable(ctx, dy):
         if spec.act in (ACT_TANH, ACT_SIGMOID):
             raise NotImplementedError("b200gan: double backward through Dropout2d fused with tanh / sigmoid")
     dx = ConvDgradFn.apply(dz, weight, g) if ctx.needs_input_grad[0] else None
+    if dx is not None and ctx.in_nchw:
+        dx = ToContiguousFn.apply(dx)   # the layout of the input: a script may .view() its gradient (dualgan.py:130)
     dw = ConvWgradFn.apply(x, dz, g, tuple(weight.shape)) if ctx.needs_input_grad[1] else None
     db = dz.sum((0, 2, 3)) if (ctx.has_bias and ctx.needs_input_grad[2]) else None
     return dx, dw, db, None, None, None
@@ -281,6 +284,7 @@ class NormFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, gamma, beta, stats, running_mean, running_var, nbt, spec: NormSpec):
         ops._require_cuda(x, "norm input")
+        x_in = x
         x = _as_cl(x)
         if stats is not None and stats.numel() == 0:
             stats = None
@@ -294,14 +298,30 @@ class NormFn(torch.autograd.Function):
         mask_from_x = (ops.Config.norm_fast and spec.act in (ACT_LRELU, ACT_RELU) and c_ % 4 == 0 and c_ // 4 <= 256
                        and 256 % (c_ // 4) == 0)
         need_y = spec.act != ACT_NONE and not mask_from_x
-        ctx.save_for_backward(x, y if need_y else None, mean_rstd, gamma, scale_shift if mask_from_x else None)
+        ctx.mask_from_x = mask_from_x
+        ctx.x_is_input = x is x_in  # else the saved x has no autograd history (create_graph needs it)
+        # scale_shift is always kept: the double backward recomputes the activation mask from it
+        ctx.save_for_backward(x, y if need_y else None, mean_rstd, gamma, scale_shift)
         return y
 
     @staticmethod
-    @torch.autograd.function.once_differentiable
     def backward(ctx, dy):
         x, y, mean_rstd, gamma, scale_shift = ctx.saved_tensors
         spec = ctx.spec
+        if torch.is_grad_enabled():
+            # autograd.grad(..., create_graph=True): the gradient penalty of a BatchNorm critic (dragan.py:144-167,
+            # dualgan.py:116-135) differentiates THROUGH this backward
+            if spec.per_sample:
+                raise NotImplementedError("b200gan: double backward through InstanceNorm2d")
+            if spec.act not in (ACT_NONE, ACT_LRELU, ACT_RELU):
+                raise NotImplementedError("b200gan: double backward through a norm with a fused tanh / sigmoid")
+            if not ctx.x_is_input:
+                raise NotImplementedError("b200gan: double backward through a norm whose input was not channels_last")
+            dx, dgamma, dbeta = NormBwdFn.apply(dy, x, gamma, y, mean_rstd, scale_shift, spec, ctx.mask_from_x)
+            want_params = gamma is not None
+            return (dx, dgamma if want_params and ctx.needs_input_grad[1] else None,
+                    dbeta if want_params and ctx.needs_input_grad[2] else None, None, None, None, None, None)
+        scale_shift = scale_shift if ctx.mask_from_x else None
         dy = _as_cl(dy)
         need_params = gamma is not None and (ctx.needs_input_grad[1] or ctx.needs_input_grad[2])
         dx, dgb = ops.norm_backward(dy, x, y, mean_rstd, None if gamma is None else gamma.detach(), spec.per_sample,
@@ -314,6 +334,40 @@ class NormFn(torch.autograd.Function):
             if spec.per_sample:  # affine InstanceNorm2d: parameters are shared across samples
                 dgamma, dbeta = dgamma.view(n, c).sum(0), dbeta.view(n, c).sum(0)
         return dx, dgamma, dbeta, None, None, None, None, None
+
+
+class NormBwdFn(torch.autograd.Function):
+    """The first-order backward of a training-mode BatchNorm2d [+ LeakyReLU / ReLU] as a differentiable node:
+    (dy, x, gamma) -> (dx, dgamma, dbeta), with y / mean_rstd / scale_shift / spec as constants.  Forward is the same
+    kernel as NormFn.backward (b200gan_norm_bwd); backward is b200gan_norm_bwd_bwd.  mask_from_x: the first-order kernel
+    takes the activation mask from scale_shift (else from the saved output y), exactly as NormFn.backward chose."""
+
+    @staticmethod
+    def forward(ctx, dy, x, gamma, y, mean_rstd, scale_shift, spec: NormSpec, mask_from_x):
+        x = _as_cl(x.detach())
+        g = None if gamma is None else gamma.detach()
+        dx, dgb = ops.norm_backward(_as_cl(dy.detach()), x, None if y is None else y.detach(), mean_rstd, g, False,
+                                    spec.eps, spec.act, spec.slope, True, spec.rtf_dx,
+                                    scale_shift if mask_from_x else None)
+        c = x.shape[1]
+        ctx.spec = spec
+        ctx.set_materialize_grads(False)
+        ctx.save_for_backward(dy, x, gamma, mean_rstd, scale_shift)
+        return dx, dgb[:c].clone(), dgb[c:].clone()  # two outputs, not two views of one buffer
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, u, gg_gamma, gg_beta):
+        dy, x, gamma, mean_rstd, scale_shift = ctx.saved_tensors
+        spec = ctx.spec
+        dy = _as_cl(dy)
+        u = torch.zeros_like(dy, memory_format=ops.CL) if u is None else _as_cl(u)
+        need_dgamma = gamma is not None and ctx.needs_input_grad[2]
+        gx, gdy, dgamma = ops.norm_backward_backward(
+            dy, x, u, mean_rstd, scale_shift, None if gamma is None else gamma.detach(),
+            None if gg_gamma is None or gamma is None else gg_gamma.contiguous(),
+            None if gg_beta is None or gamma is None else gg_beta.contiguous(), spec.eps, spec.act, spec.slope, need_dgamma)
+        return gdy, gx, dgamma, None, None, None, None, None
 
 
 @dataclass(frozen=True)
@@ -475,6 +529,25 @@ class NbSpec:
     groups: int = 1           # statistics groups of the batch (ops.bn_groups)
 
 
+def _bn_edge_differentiable(a, gamma, beta, edge, want_xhat=True):
+    """The BatchNorm of a chain edge as differentiable nodes, for a create_graph backward: the normalised tensor
+    BN(a) (a NormFn of (a, gamma, beta); None unless want_xhat) and a function mapping a gradient w.r.t. BN(a) to
+    (gradient w.r.t. the stored a, dgamma, dbeta) through NormBwdFn.  Both use the batch sums the forward kept in edge.stats; norm_finalize consumes
+    (zeroes) the sums it is given, so each call gets a copy.  The running statistics are not touched (the forward
+    already updated them once)."""
+    if edge.groups > 1:
+        raise NotImplementedError("b200gan: double backward through a grouped pass (ops.bn_groups)")
+    spec = NormSpec(eps=edge.eps)
+    xhat = NormFn.apply(a, gamma, beta, edge.stats.clone(), None, None, None, spec) if want_xhat else None
+    mean_rstd, scale_shift = ops.norm_finalize(tuple(a.shape), edge.stats.clone(), edge.gamma, edge.beta, None, None,
+                                               None, False, edge.eps, 0.0, a.device)
+
+    def backward(g_xhat):
+        return NormBwdFn.apply(g_xhat, a, gamma, None, mean_rstd, scale_shift, spec, True)
+
+    return xhat, backward
+
+
 class NbConvFn(torch.autograd.Function):
     """One layer of a fused narrow chain (csrc/narrow_block.cu): conv over the (virtually normalised) stored output of
     the previous layer, + bias, activation, Dropout2d scale, + the batch sums for the following BatchNorm.
@@ -488,6 +561,7 @@ class NbConvFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, x, weight, bias, chan_scale, in_gamma, in_beta, in_rm, in_rv, in_nbt, in_edge, out_box, spec, cache):
         ops._require_cuda(x, "conv input")
+        ctx.in_nchw = not ops.is_cl(x)
         x = _as_cl(x)
         g, _ = ops.make_geom(tuple(x.shape), tuple(weight.shape), spec.stride, (spec.pad,) * 4)
         w = weight.detach()
@@ -496,7 +570,7 @@ class NbConvFn(torch.autograd.Function):
                                 in_edge, in_rm, in_rv, in_nbt, spec.momentum, spec.want_stats, spec.groups)
         ctx.g, ctx.spec, ctx.cache, ctx.in_edge, ctx.out_box = g, spec, cache, in_edge, out_box
         ctx.has_bias = bias is not None
-        ctx.save_for_backward(x, weight, y, chan_scale)
+        ctx.save_for_backward(x, weight, y, chan_scale, in_gamma, in_beta)
         if spec.want_stats:
             ctx.mark_non_differentiable(stats)
             return y, stats
@@ -504,15 +578,22 @@ class NbConvFn(torch.autograd.Function):
 
     @staticmethod
     def backward(ctx, gy, *unused):
-        x, weight, y, chan_scale = ctx.saved_tensors
+        x, weight, y, chan_scale, in_gamma, in_beta = ctx.saved_tensors
         g, spec, in_edge = ctx.g, ctx.spec, ctx.in_edge
         out_edge = ctx.out_box[0] if ctx.out_box else None
-        if torch.is_grad_enabled():
+        create_graph = torch.is_grad_enabled()
+        # A chain that has been through a create_graph backward stays in the stored protocol for every later backward
+        # (the penalty's .backward() reaches these forward nodes with gradients w.r.t. the stored tensors)
+        stored = create_graph or any(e is not None and e.grad_of_stored for e in (in_edge, out_edge))
+        if stored:
             # autograd.grad(..., create_graph=True) through a chain: the gradient penalty of a conv critic (SURVEY.md 8f
-            # N2; critics carry no BatchNorm, stargan/models.py:87-115).  Same differentiable nodes as ConvFn.
-            if in_edge is not None or out_edge is not None:
-                raise NotImplementedError("b200gan: double backward through a fused conv chain with BatchNorm2d; set "
-                                          "B200GAN_FUSE_CHAIN=0 for this model")
+            # N2: stargan/models.py:87-115, and with BatchNorm dragan.py:144-167).  Same differentiable nodes as ConvFn;
+            # across a BatchNorm edge every gradient is w.r.t. the STORED tensor (BnEdge.grad_of_stored).
+            if spec.groups > 1:
+                raise NotImplementedError("b200gan: double backward through a grouped pass (ops.bn_groups)")
+            if out_edge is not None and not out_edge.grad_of_stored:
+                raise RuntimeError("b200gan: fused conv chain: the consumer of this layer did not run its create_graph "
+                                   "backward first")
             dz = gy
             if spec.act == ACT_LRELU:
                 dz = dz * torch.where(y > 0, 1.0, spec.slope)
@@ -520,10 +601,22 @@ class NbConvFn(torch.autograd.Function):
                 dz = dz * (y > 0).to(gy.dtype)
             if chan_scale is not None:
                 dz = dz * chan_scale.view(chan_scale.shape[0], chan_scale.shape[1], 1, 1)
-            gx = ConvDgradFn.apply(dz, weight, g) if ctx.needs_input_grad[0] else None
-            dw = ConvWgradFn.apply(x, dz, g, tuple(weight.shape)) if ctx.needs_input_grad[1] else None
+            xin = x
+            if in_edge is not None:
+                in_edge.grad_of_stored = True
+                xin, norm_bwd = _bn_edge_differentiable(x, in_gamma, in_beta, in_edge, ctx.needs_input_grad[1])
+            need_params = in_edge is not None and (ctx.needs_input_grad[4] or ctx.needs_input_grad[5])
+            gx = dgamma = dbeta = None
+            if ctx.needs_input_grad[0] or need_params:
+                gx = ConvDgradFn.apply(dz, weight, g)
+                if in_edge is not None:
+                    gx, dgamma, dbeta = norm_bwd(gx)
+                elif ctx.in_nchw:
+                    gx = ToContiguousFn.apply(gx)
+            dw = ConvWgradFn.apply(xin, dz, g, tuple(weight.shape)) if ctx.needs_input_grad[1] else None
             db = dz.sum((0, 2, 3)) if (ctx.has_bias and ctx.needs_input_grad[2]) else None
-            return (gx, dw, db) + (None,) * 10
+            return (gx, dw, db, None, dgamma if ctx.needs_input_grad[4] else None,
+                    dbeta if ctx.needs_input_grad[5] else None) + (None,) * 7
         gy, y, x = gy.detach(), y.detach(), x.detach()
         if out_edge is not None and out_edge.sums is None:
             raise RuntimeError("b200gan: fused conv chain: the consumer of this layer did not run its backward first")
@@ -558,13 +651,22 @@ class NbTailFn(torch.autograd.Function):
         a = _as_cl(a)
         out = ops.nb_tail_fwd(a, edge, rm, rv, nbt, momentum, nchw)
         ctx.edge, ctx.nchw = edge, nchw
-        ctx.save_for_backward(a)
+        ctx.save_for_backward(a, gamma, beta)
         return out
 
     @staticmethod
-    @torch.autograd.function.once_differentiable
     def backward(ctx, dout):
-        (a,) = ctx.saved_tensors
+        a, gamma, beta = ctx.saved_tensors
+        if torch.is_grad_enabled() or ctx.edge.grad_of_stored:
+            # create_graph=True (dragan.py:144-167), and every later backward of the same forward: the gradient handed
+            # to the producer is w.r.t. the stored a
+            ctx.edge.grad_of_stored = True
+            if not ops.is_cl(dout):
+                dout = ToChannelsLastFn.apply(dout.contiguous())
+            _, norm_bwd = _bn_edge_differentiable(a, gamma, beta, ctx.edge, want_xhat=False)
+            g, dgamma, dbeta = norm_bwd(dout)
+            return (g, dgamma if ctx.needs_input_grad[1] else None, dbeta if ctx.needs_input_grad[2] else None,
+                    None, None, None, None, None, None)
         dout = dout.contiguous() if ctx.nchw else _as_cl(dout)
         g, sums = ops.nb_tail_bwd(a, ctx.edge, dout, ctx.nchw)
         ctx.edge.sums = sums

@@ -332,6 +332,27 @@ def norm_backward(dy, x, y, mean_rstd, gamma, per_sample, eps, act=ACT_NONE, slo
     return dx, dgb
 
 
+def norm_backward_backward(dy, x, u, mean_rstd, scale_shift, gamma, gg_gamma, gg_beta, eps, act=ACT_NONE, slope=0.0,
+                           need_dgamma=False):
+    """Double backward of training-mode BatchNorm2d [+ LeakyReLU / ReLU]: given u = dL/d(dx) and (optionally) dL/d(dgamma),
+    dL/d(dbeta) for the outputs of norm_backward(dy, x, ...), returns (dL/dx, dL/d(dy), dL/dgamma or None).  All of dy, x,
+    u are NHWC; scale_shift carries the activation mask (required with an activation)."""
+    for t_ in (dy, x, u):
+        if not is_cl(t_):
+            raise RuntimeError("b200gan norm_backward_backward: NHWC (channels_last) tensors expected")
+    lib = _lib.load()
+    d = _norm_desc(x, False, eps, 0.0, act, slope, False)
+    c = x.shape[1]
+    sums = zero_scratch(x.device, 5 * c)
+    gx = torch.empty_like(x, memory_format=CL)
+    gdy = torch.empty_like(x, memory_format=CL)
+    dgamma = torch.empty(c, device=x.device, dtype=torch.float32) if need_dgamma else None
+    _lib.check(lib.b200gan_norm_bwd_bwd(ctypes.byref(d), dy.data_ptr(), x.data_ptr(), u.data_ptr(), mean_rstd.data_ptr(),
+                                        _ptr(scale_shift), _ptr(gamma), _ptr(gg_gamma), _ptr(gg_beta), sums.data_ptr(),
+                                        gx.data_ptr(), gdy.data_ptr(), _ptr(dgamma), _stream()), "norm_bwd_bwd")
+    return gx, gdy, dgamma
+
+
 # ---- shape ops ------------------------------------------------------------------------------------
 def upsample2x(x):
     n, c, h, w = x.shape
@@ -378,13 +399,17 @@ def act_forward(x, act, slope, mask=None, mask_per_channel=False):
 # ---- Discriminator conv blocks as a fused chain (csrc/narrow_block.cu) ------------------------------------------
 class BnEdge:
     """A training-mode BatchNorm2d between two fused convs: its batch statistics (fp64 sums of the producer's output)
-    and parameters.  `sums` is filled by the consumer's backward (sum g, sum g * ahat) for the producer's backward."""
+    and parameters.  `sums` is filled by the consumer's backward (sum g, sum g * ahat) for the producer's backward.
+    `grad_of_stored` is set by the consumer's backward when it runs under create_graph: from then on every backward
+    through this edge hands the producer a gradient w.r.t. the stored tensor a (the BatchNorm backward already done);
+    while it is False the gradient is w.r.t. the virtual normalised tensor and `sums` completes it."""
 
     def __init__(self, stats, gamma, beta, eps, count, groups=1):
         """stats: [groups][2][C] fp64; count: elements per channel and group (see b200gan_nb_bn in include/b200gan.h)."""
         self.stats, self.gamma, self.beta, self.eps, self.count = stats, gamma, beta, float(eps), float(count)
         self.groups = int(groups)
         self.sums = None
+        self.grad_of_stored = False
 
     def c_struct(self):
         b = NbBn()

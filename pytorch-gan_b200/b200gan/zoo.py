@@ -130,6 +130,29 @@ class WGANGPDiscriminator(tnn.Module):
         return self.model(img.view(img.shape[0], -1))
 
 
+class DualGANDiscriminator(tnn.Module):
+    """dualgan/models.py:102-123: a WGAN-GP critic with BatchNorm2d(out, 0.8) + LeakyReLU(0.2) blocks and a patch head
+    (ZeroPad2d((1, 0, 1, 0)) -> Conv2d(256, 1, 4)); its gradient penalty (dualgan.py:116-135) differentiates through the
+    BatchNorm backward."""
+
+    def __init__(self, in_channels=3, nn=None):
+        super().__init__()
+        nn = nn or namespace()
+
+        def block(i, o, normalize=True):
+            layers = [nn.Conv2d(i, o, 4, stride=2, padding=1)]
+            if normalize:
+                layers.append(nn.BatchNorm2d(o, 0.8))
+            layers.append(nn.LeakyReLU(0.2, inplace=True))
+            return layers
+
+        self.model = nn.Sequential(*block(in_channels, 64, normalize=False), *block(64, 128), *block(128, 256),
+                                   nn.ZeroPad2d((1, 0, 1, 0)), nn.Conv2d(256, 1, kernel_size=4))
+
+    def forward(self, img):
+        return self.model(img)
+
+
 # ------------------------------------------------------------------------------------------------
 # Pix2Pix (BASELINE config 3): pix2pix/models.py:20-133
 # ------------------------------------------------------------------------------------------------
